@@ -362,6 +362,22 @@ def run_dressing(args):
                                    'note': 'algorithmic bytes = 190 KB per env and substep (SURVEY.md 8(d)); the kernel keeps the cloth in shared memory over the 8 substeps of a launch, so its DRAM traffic is ~1/8 of that'}}))
 
 
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each per-env output array (rows = envs) as `out_dir/<name>.npy` in float32.  Above DUMP_BYTES in all, the same
+    fixed, seeded sample of envs (sorted) is taken from every array, so two runs with the same arguments stay comparable."""
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(4 * a[0].size for a in arrays.values())
+    rows = np.arange(n)
+    if n * row_bytes > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(n, DUMP_BYTES // row_bytes, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), np.ascontiguousarray(a[rows], dtype=np.float32))
+
+
 def ncu_traffic(kernel):
     """DRAM bytes (read + write) of one launch of `kernel` from the newest committed `ncu --set full` summary
     (profiles/r*_ncu_<kernel>.csv, written by tools/ncu_summary.py); (None, None) if there is none."""
@@ -408,7 +424,14 @@ def main():
     ap.add_argument('--action-scale', type=float, default=0.2, help='bedbathing: scale of the random actions (small actions keep the pad on the skin)')
     ap.add_argument('--toc-attempts', type=int, default=10, help='dressing / bedbathing: random base poses ranked per reset (the reference uses 50)')
     ap.add_argument('--sub-batches', type=int, default=int(os.environ.get('AG_SUB_BATCHES', '1')), help='independent sub-batches per GPU, each on its own stream')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='feeding: write obs / reward / done / info of the last timed step (rank 0) as DIR/<name>.npy, float32; '
+                         'above 64 MB a fixed, seeded sample of envs')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.workload != 'feeding' or args.impl == 'reference'):
+        ap.error('--dump-outputs covers the device path of the feeding workload only')
     if args.workload == 'bedbathing':
         return run_bedbathing(args)
     if args.workload == 'dressing':
@@ -519,6 +542,8 @@ def main():
     elapsed_ms = float(t.item())
     value = world * n * K / (elapsed_ms / 1000.0)
     rew_value_path = rew.detach().cpu().numpy().copy()        # reward of the last timed step (compared with the e2e path below)
+    # the later passes step on in the same buffers: keep what the last timed step handed back
+    last_step = {'obs': obs.cpu().numpy(), 'reward': rew_value_path, 'done': done.cpu().numpy(), 'info': info.cpu().numpy()} if args.dump_outputs else None
     # the same K steps timed back to back (no flush, no per-step sync): how much the pipeline overlap is worth
     torch.cuda.synchronize()
     with torch.cuda.stream(stream):
@@ -622,6 +647,8 @@ def main():
             out['cpu_baseline'] = {'value': v, 'unit': 'env-steps/s', 'cores': cores, 'kind': 'port',
                                    'sample': '%d envs x %d env-steps (%.2f s wall, %.0f core-seconds), CPU restatement (PyBullet unavailable), %d threads (affinity / cgroup quota)' % (ne, ns, tsec, tsec * cores, cores),
                                    'one_thread': {'value': v1, 'cores': 1, 'sample': '64 envs x %d env-steps (%.2f s)' % (ns, t1)}}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last_step)
         print(json.dumps(out))
     if world > 1:
         dist.destroy_process_group()

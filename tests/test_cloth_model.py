@@ -1,5 +1,6 @@
 """Cloth template (assistive_gym_b200/cloth.py, tools/compile_assets.compile_cloth): pins against constants the reference
 embeds in envs/dressing.py, and structural invariants the CUDA kernel relies on."""
+import json
 import os
 
 import numpy as np
@@ -9,7 +10,7 @@ from assistive_gym_b200.cloth import ClothModel
 from assistive_gym_b200.dressing_batch import (CLOTH_ANCHORS, CLOTH_ORIG_POS, CLOTH_POSITION, CLOTH_SCALE, TRIANGLE1, TRIANGLE2)
 from assistive_gym_b200.scene import quat_from_rpy
 
-REF_OBJ = '/root/reference/assistive_gym/envs/assets/clothing/hospitalgown_reduced.obj'
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'reference_assets.json')
 
 
 @pytest.fixture(scope='module')
@@ -30,10 +31,10 @@ def test_node_numbering_and_placement_pinned_by_reference_constants(gown):
     assert np.linalg.norm(ring.mean(axis=0) - CLOTH_ORIG_POS) < 0.2
     x_unscaled = gown.place(CLOTH_POSITION, quat_from_rpy([0, 0, np.pi]))
     assert np.linalg.norm(x_unscaled[CLOTH_ANCHORS] - CLOTH_ORIG_POS, axis=1).min() > 0.2
-    if os.path.exists(REF_OBJ):                                  # `v`-line order scatters the same indices over the gown
-        v = np.array([[float(t) for t in l.split()[1:4]] for l in open(REF_OBJ) if l.startswith('v ')]) * CLOTH_SCALE
-        assert np.ptp(v[TRIANGLE1 + TRIANGLE2], axis=0).max() > 0.5
-        assert len(v) == gown.n_nodes == 3966
+    obj = json.load(open(GOLDEN))['gown_obj']                   # the reference's .obj: `v`-line order scatters the same indices over the gown
+    assert obj['indices'] == TRIANGLE1 + TRIANGLE2
+    assert np.ptp(np.array(obj['vertices']) * CLOTH_SCALE, axis=0).max() > 0.5
+    assert obj['n_vertices'] == gown.n_nodes == 3966
 
 
 def test_link_colouring_is_a_proper_edge_colouring_in_list_order(gown):

@@ -158,14 +158,12 @@ def test_realistic_joint_limit_classifier():
 
 
 def test_keras_file_compiles_to_the_committed_weights():
-    """tools/compile_assets.py reads the reference's HDF5 file with its own minimal reader (no h5py in this image); skipped on boxes
-    without the reference tree."""
+    """tools/compile_assets.py reads the reference's HDF5 file (an unchanged copy under tests/golden) with its own minimal reader
+    (no h5py needed)."""
     import os
     import sys
-    ref = '/root/reference/assistive_gym/envs/assets/realistic_arm_limits_model.h5'
-    if not os.path.exists(ref):
-        pytest.skip('reference assets not present')
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    ref = os.path.join(root, 'tests', 'golden', 'realistic_arm_limits_model.h5')
     sys.path.insert(0, os.path.join(root, 'tools'))
     from compile_assets import compile_keras_mlp
     from assistive_gym_b200.limits_model import load_model

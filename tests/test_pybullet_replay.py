@@ -17,8 +17,8 @@ gym = pytest.importorskip('gym')
 
 
 def _reference_env():
-    ref = os.environ.get('AG_REFERENCE_PATH', '/root/reference')
-    if not os.path.isdir(os.path.join(ref, 'assistive_gym')):
+    ref = os.environ.get('AG_REFERENCE_PATH')
+    if not ref or not os.path.isdir(os.path.join(ref, 'assistive_gym')):
         pytest.skip('reference package not found (set AG_REFERENCE_PATH)')
     sys.path.insert(0, ref)
     for m in [m for m in sys.modules if m == 'assistive_gym' or m.startswith('assistive_gym.')]:

@@ -1,12 +1,11 @@
 """The scene description both the product and the oracle consume, checked against sources neither of them shares:
   * the compiled robot models (assets/*.agmodel.json, written by tools/compile_assets.py) against the reference's URDF files read
-    here with a separate, minimal XML walk (skipped where /root/reference is absent: the GPU box);
+    with a separate, minimal XML walk (tests/golden/make_golden_reference_assets.py; its output is tests/golden/reference_assets.json);
   * masses, joint frames, axes and limits of the finalized scene arrays against the same XML;
   * inertia-from-shape of single primitives against the closed forms (sphere 2/5 m r^2; anything else: the box of the shape's
     bounding box, which is what Bullet's compound / createMultiBody path uses -- recalled, DESIGN.md section 5)."""
 import json
 import os
-import xml.etree.ElementTree as ET
 
 import numpy as np
 import pytest
@@ -14,49 +13,24 @@ import pytest
 from assistive_gym_b200.scene import SceneBuilder
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_ASSETS = '/root/reference/assistive_gym/envs/assets'
-URDFS = {'jaco': 'jaco/j2s7s300_gym.urdf', 'sawyer': 'sawyer/sawyer.urdf', 'pr2': 'PR2/pr2_no_torso_lift_tall.urdf'}
+ROBOTS = ('jaco', 'pr2', 'sawyer')
 
 
-def _floats(s, n, default=0.0):
-    v = [float(x) for x in s.split()] if s else []
-    return v + [default] * (n - len(v))
+def _stored_urdf_walk(name):
+    """child link name -> (joint name, type, parent link, xyz, rpy, axis, lower, upper), link name -> (mass, com xyz, has <inertial>)"""
+    u = json.load(open(os.path.join(ROOT, 'tests', 'golden', 'reference_assets.json')))['urdf'][name]
+    return u['joints'], u['links']
 
 
-def _walk_urdf(path):
-    """child link name -> (joint name, type, parent link, xyz, rpy, axis, lower, upper), link name -> (mass, com xyz)"""
-    root = ET.parse(path).getroot()
-    joints, links = {}, {}
-    for j in root.findall('joint'):
-        o, a, lim = j.find('origin'), j.find('axis'), j.find('limit')
-        joints[j.find('child').get('link')] = (
-            j.get('name'), j.get('type'), j.find('parent').get('link'),
-            _floats(o.get('xyz') if o is not None else '', 3), _floats(o.get('rpy') if o is not None else '', 3),
-            _floats(a.get('xyz'), 3) if a is not None else [1.0, 0.0, 0.0],
-            float(lim.get('lower', 0.0)) if lim is not None else 0.0, float(lim.get('upper', 0.0)) if lim is not None else 0.0)
-    for l in root.findall('link'):
-        i = l.find('inertial')
-        m, c = 0.0, [0.0, 0.0, 0.0]
-        if i is not None:
-            m = float(i.find('mass').get('value'))
-            o = i.find('origin')
-            c = _floats(o.get('xyz') if o is not None else '', 3)
-        links[l.get('name')] = (m, c)
-    return joints, links
-
-
-@pytest.mark.parametrize('name', sorted(URDFS))
+@pytest.mark.parametrize('name', ROBOTS)
 def test_compiled_model_matches_the_urdf(name):
-    path = os.path.join(REF_ASSETS, URDFS[name])
-    if not os.path.exists(path):
-        pytest.skip('reference assets not present')
-    joints, links = _walk_urdf(path)
+    joints, links = _stored_urdf_walk(name)
     m = json.load(open(os.path.join(ROOT, 'assistive_gym_b200', 'assets', name + '.agmodel.json')))
     assert len(m['links']) == len(links)
     seen = set()
     for k, lk in enumerate(m['links']):
         seen.add(lk['name'])
-        mass, com = links[lk['name']]
+        mass, com, _ = links[lk['name']]
         assert abs(lk['inertial']['mass'] - mass) < 1e-12 and np.allclose(lk['inertial']['com_xyz'], com, atol=1e-12), lk['name']
         if lk['name'] not in joints:                      # the root link
             assert lk['parent'] < 0
@@ -73,10 +47,7 @@ def test_compiled_model_matches_the_urdf(name):
 
 
 def test_scene_arrays_of_the_jaco_match_the_urdf():
-    path = os.path.join(REF_ASSETS, URDFS['jaco'])
-    if not os.path.exists(path):
-        pytest.skip('reference assets not present')
-    joints, links = _walk_urdf(path)
+    joints, links = _stored_urdf_walk('jaco')
     b = SceneBuilder()
     body = b.load_urdf('jaco', base_pos=[0.3, -0.1, 0.7], fixed_base=True)
     names = [lk.name for lk in b.links if lk.body == body]
@@ -85,8 +56,7 @@ def test_scene_arrays_of_the_jaco_match_the_urdf():
     assert int(sc['body_nlinks'][body]) == len(links) == len(names)
     for i, nm in enumerate(names):
         k = l0 + i
-        mass, com = links[nm]
-        has_inertial = ET.parse(path).getroot().find("link[@name='%s']/inertial" % nm) is not None
+        mass, com, has_inertial = links[nm]
         # a link without <inertial> gets Bullet's default mass 1 (its URDF importer's fallback); the base is held by `fixed_base`, whatever its mass
         assert abs(float(sc['link_mass'][k]) - (mass if has_inertial else 1.0)) < 1e-9, nm
         if nm not in joints:
