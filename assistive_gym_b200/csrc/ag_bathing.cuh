@@ -16,26 +16,10 @@ struct BathDev {
   int n_slots;                    // max colliders of a person
 };
 
-// action -> PD targets (env.py:187-217), same accumulate-with-limit-clamp rule as the feeding path
+// action -> PD targets (env.py:187-217)
 AG_HDN inline void bathing_pre_body(int e, const SimDev& S, const KP& p) {
-  const int N = S.N;
   const BathDev& B = *(const BathDev*)p.p1;
-  const float* act = (const float*)p.p0 + (size_t)e * 7;
-  B.iteration[e] += 1;
-  for (int j = 0; j < 7; j++) {
-    float raw = act[j];
-    B.action[(size_t)j * N + e] = raw;
-    float a = clampf(raw, -1.f, 1.f) * B.P.action_multiplier;
-    int k = B.P.arm_links[j];
-    float q = ld1(S.jq, k, N, e);
-    float lo = B.P.arm_lower[j], hi = B.P.arm_upper[j];
-    for (int s = 0; s < B.P.frame_skip; s++) {
-      if (q + a < lo) { a = 0.f; q = lo; }
-      if (q + a > hi) { a = 0.f; q = hi; }
-      q += a;
-    }
-    st1(S.motor_target, k, N, e, q);
-  }
+  take_step(e, S, (const float*)p.p0, B.iteration, B.action, B.P.arm_links, B.P.arm_lower, B.P.arm_upper, B.P.action_multiplier, B.P.frame_skip);
 }
 
 // thread = (collider slot of the person, env): distance from that collider to the nearest wiper collider,

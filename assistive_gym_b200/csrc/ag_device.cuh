@@ -39,6 +39,37 @@ AG_HD q4 tv4(const float* p, int i) { return q4(AG_LDG(p + 4 * i), AG_LDG(p + 4 
 AG_HD float cf_ld(const float* d, int slot, int f, int N, int e) { return d[((size_t)slot * AG_CF + f) * N + e]; }
 AG_HD void cf_st(float* d, int slot, int f, int N, int e, float v) { d[((size_t)slot * AG_CF + f) * N + e] = v; }
 
+// ------------------------------------------------------------------ the fused env steps' shared action handling
+// AssistiveEnv.take_step (env.py:187-217): counts the env step, keeps the raw action ([7][N], for the action penalty) and drives
+// the robot's 7 arm joints to PD targets: the clipped, scaled action accumulated frame_skip times onto the joint angle, with
+// the limit clamp of every accumulation.  `actions` is the step's [N][7] env-major input.
+AG_HD void take_step(int e, const SimDev& S, const float* actions, int* iteration, float* action, const int* arm_links,
+                     const float* arm_lower, const float* arm_upper, float action_multiplier, int frame_skip) {
+  const int N = S.N;
+  const float* act = actions + (size_t)e * 7;
+  iteration[e] += 1;
+  for (int j = 0; j < 7; j++) {
+    float raw = act[j];
+    action[(size_t)j * N + e] = raw;
+    float a = clampf(raw, -1.f, 1.f) * action_multiplier;
+    int k = arm_links[j];
+    float q = ld1(S.jq, k, N, e);
+    float lo = arm_lower[j], hi = arm_upper[j];
+    for (int s = 0; s < frame_skip; s++) {
+      if (q + a < lo) { a = 0.f; q = lo; }
+      if (q + a > hi) { a = 0.f; q = hi; }
+      q += a;
+    }
+    st1(S.motor_target, k, N, e, q);
+  }
+}
+// tremor (env.py:212-215): the person's `nj` joints are driven to rest +- amplitude ([nj][N]), the sign flips every env step
+AG_HD void tremor_step(int e, const SimDev& S, int nj, const int* joints, int iteration, const float* rest, const float* amp) {
+  const int N = S.N;
+  float sgn = (iteration % 2 == 0) ? 1.f : -1.f;
+  for (int j = 0; j < nj; j++) st1(S.motor_target, joints[j], N, e, rest[(size_t)j * N + e] + sgn * amp[(size_t)j * N + e]);
+}
+
 // plane k of collider (local) -> (n, d)
 AG_HD void ld_plane(const float* planes, int k, f3& n, float& d) {
   n = f3(AG_LDG(planes + 4 * k), AG_LDG(planes + 4 * k + 1), AG_LDG(planes + 4 * k + 2)); d = AG_LDG(planes + 4 * k + 3);

@@ -18,31 +18,11 @@ struct DressDev {
 
 // action -> PD targets of the robot's 7 arm joints (env.py:187-217)
 AG_HDN inline void dressing_pre_body(int e, const SimDev& S, const KP& p) {
-  const int N = S.N;
   const DressDev& D = *(const DressDev*)p.p1;
-  const float* act = (const float*)p.p0 + (size_t)e * 7;
-  D.iteration[e] += 1;
-  for (int j = 0; j < 7; j++) {
-    float raw = act[j];
-    D.action[(size_t)j * N + e] = raw;
-    float a = clampf(raw, -1.f, 1.f) * D.P.action_multiplier;
-    int k = D.P.arm_links[j];
-    float q = ld1(S.jq, k, N, e);
-    float lo = D.P.arm_lower[j], hi = D.P.arm_upper[j];
-    for (int s = 0; s < D.P.frame_skip; s++) {
-      if (q + a < lo) { a = 0.f; q = lo; }
-      if (q + a > hi) { a = 0.f; q = hi; }
-      q += a;
-    }
-    st1(S.motor_target, k, N, e, q);
-  }
-  // a tremor human is an agent (env.py:130): its arm targets flip sign around the rest pose every env step (env.py:212-215)
-  if (D.tremor_on[e]) {
-    bool male = D.male[e] != 0;
-    float sgn = (D.iteration[e] % 2 == 0) ? 1.f : -1.f;
-    for (int j = 0; j < 10; j++)
-      st1(S.motor_target, male ? D.P.human_arm_m[j] : D.P.human_arm_f[j], N, e, D.tremor_rest[(size_t)j * N + e] + sgn * D.tremor_amp[(size_t)j * N + e]);
-  }
+  take_step(e, S, (const float*)p.p0, D.iteration, D.action, D.P.arm_links, D.P.arm_lower, D.P.arm_upper, D.P.action_multiplier, D.P.frame_skip);
+  // a tremor human is an agent (env.py:130): its arm targets flip sign around the rest pose every env step
+  if (D.tremor_on[e])
+    tremor_step(e, S, 10, D.male[e] ? D.P.human_arm_m : D.P.human_arm_f, D.iteration[e], D.tremor_rest, D.tremor_amp);
 }
 
 AG_HD float dress_sign(float v) { return v > 0.f ? 1.f : (v < 0.f ? -1.f : 0.f); }

@@ -146,33 +146,11 @@ AG_HDN inline void closest_body(int e, const SimDev& S, const KP& p) {
 // ------------------------------------------------------------------ fused FeedingEnv
 // action -> PD targets.  p0 = action [N][7] (env-major), p1 = FeedDev*
 AG_HDN inline void feeding_pre_body(int e, const SimDev& S, const KP& p) {
-  const int N = S.N;
   const FeedDev& F = *(const FeedDev*)p.p1;
-  const float* act = (const float*)p.p0 + (size_t)e * 7;
-  F.iteration[e] += 1;
-  for (int j = 0; j < 7; j++) {
-    float raw = act[j];
-    F.action[(size_t)j * N + e] = raw;
-    float a = clampf(raw, -1.f, 1.f) * F.P.action_multiplier;
-    int k = F.P.arm_links[j];
-    float q = ld1(S.jq, k, N, e);
-    float lo = F.P.arm_lower[j], hi = F.P.arm_upper[j];
-    for (int s = 0; s < F.P.frame_skip; s++) {
-      if (q + a < lo) { a = 0.f; q = lo; }
-      if (q + a > hi) { a = 0.f; q = hi; }
-      q += a;
-    }
-    st1(S.motor_target, k, N, e, q);
-  }
-  // tremor (env.py:212-215): the head joints are driven to rest +- amplitude, sign flips every env step
-  if (F.tremor_on[e]) {
-    bool male = F.male[e] != 0;
-    float sgn = (F.iteration[e] % 2 == 0) ? 1.f : -1.f;
-    for (int j = 0; j < 4; j++) {
-      int k = male ? F.P.head_joints_m[j] : F.P.head_joints_f[j];
-      st1(S.motor_target, k, N, e, F.tremor_rest[(size_t)j * N + e] + sgn * F.tremor_amp[(size_t)j * N + e]);
-    }
-  }
+  take_step(e, S, (const float*)p.p0, F.iteration, F.action, F.P.arm_links, F.P.arm_lower, F.P.arm_upper, F.P.action_multiplier, F.P.frame_skip);
+  // tremor: the head joints
+  if (F.tremor_on[e])
+    tremor_step(e, S, 4, F.male[e] ? F.P.head_joints_m : F.P.head_joints_f, F.iteration[e], F.tremor_rest, F.tremor_amp);
 }
 
 // thread = (food i, env e): is any spoon collider within 0.1 of the food sphere? (feeding.py:71)

@@ -16,24 +16,8 @@ struct ScratchDev {
 };
 
 AG_HDN inline void scratch_pre_body(int e, const SimDev& S, const KP& p) {
-  const int N = S.N;
   const ScratchDev& D = *(const ScratchDev*)p.p1;
-  const float* act = (const float*)p.p0 + (size_t)e * 7;
-  D.iteration[e] += 1;
-  for (int j = 0; j < 7; j++) {
-    float raw = act[j];
-    D.action[(size_t)j * N + e] = raw;
-    float a = clampf(raw, -1.f, 1.f) * D.P.action_multiplier;
-    int k = D.P.arm_links[j];
-    float q = ld1(S.jq, k, N, e);
-    float lo = D.P.arm_lower[j], hi = D.P.arm_upper[j];
-    for (int s = 0; s < D.P.frame_skip; s++) {
-      if (q + a < lo) { a = 0.f; q = lo; }
-      if (q + a > hi) { a = 0.f; q = hi; }
-      q += a;
-    }
-    st1(S.motor_target, k, N, e, q);
-  }
+  take_step(e, S, (const float*)p.p0, D.iteration, D.action, D.P.arm_links, D.P.arm_lower, D.P.arm_upper, D.P.action_multiplier, D.P.frame_skip);
 }
 
 // p0 = action, p1 = ScratchDev*, p2 = obs [N][30], p3 = reward, p4 = done, p5 = info [N][4] = total force on the person, task

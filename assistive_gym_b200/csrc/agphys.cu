@@ -25,6 +25,7 @@
 #else
 #define AG_GLOBAL
 typedef void* cudaStream_t;
+enum cudaMemcpyKind { cudaMemcpyHostToDevice = 1, cudaMemcpyDeviceToHost = 2 };
 #endif
 
 static thread_local std::string g_err;
@@ -115,6 +116,22 @@ AG_KERNEL(k_cloth_snap, cloth_snap_body)
 AG_KERNEL(k_cloth_follow, cloth_follow_body)
 
 // ------------------------------------------------------------------ host object
+// The fused env steps (action -> PD targets -> frame_skip substeps -> obs / reward / done / info in one call): one record per task.
+enum FusedTask { FT_FEEDING, FT_BATHING, FT_DRESSING, FT_SCRATCH, FT_COUNT };
+static const char* const fused_name[FT_COUNT] = {"feeding", "bathing", "dressing", "scratch"};
+struct AgSim;
+typedef int (*StepEnqueue)(AgSim*, const float*, float*, float*, float*, float*);
+// CUDA-graph replay of a fused step, keyed by its device pointers
+struct StepGraph { void* exec = nullptr; const void* key[5] = {}; uint64_t launches = 0; bool valid = false; };
+struct FusedStep {
+  int obs_dim = 0;
+  StepEnqueue enqueue = nullptr;                // enqueues the task's kernels on the sim's stream
+  float *d_action = nullptr, *d_obs = nullptr, *d_reward = nullptr, *d_done = nullptr, *d_info = nullptr;   // the task's own device I/O
+  float *h_in = nullptr, *h_out = nullptr;      // pinned staging of the host-buffer step: [N][7] and [N][obs_dim + 6]
+  StepGraph graph;
+  bool ready = false;                           // the task's init has run
+};
+
 struct AgSim {
   SimDev S;
   AgConfig cfg;
@@ -129,22 +146,16 @@ struct AgSim {
   float* d_stage; size_t stage_floats;
   std::vector<float> h_stage;
   int* d_mask; int* d_links; int* d_icount;
-  // feeding
-  FeedDev F; FeedDev* F_dev; bool feeding;
-  BathDev B; BathDev* B_dev; bool bathing;
-  float *h_bpin_in, *h_bpin_out, *d_baction, *d_bobs, *d_breward, *d_bdone, *d_binfo;
-  float *d_action, *d_obs, *d_reward, *d_done, *d_info;
-  float *h_pin_in, *h_pin_out;
+  // the fused env steps' per-task state
+  FeedDev F; FeedDev* F_dev;
+  BathDev B; BathDev* B_dev;
+  DressPost DP; DressPost* DP_dev;
+  ScratchDev SD; ScratchDev* SD_dev;
+  FusedStep fused[FT_COUNT];
+  bool use_graph; int graph_failures;       // CUDA-graph replay of the fused steps
   // cloth (Dressing): one k_cloth launch per stepSimulation = `C.K` rigid substeps
   ClothDev C; ClothDev* C_dev; bool cloth; int cloth_sub, cloth_npt, cloth_qs;
-  DressPost DP; DressPost* DP_dev; bool dressing;
-  ScratchDev SD; ScratchDev* SD_dev; bool scratch;
-  float *h_spin_in, *h_spin_out, *d_saction, *d_sobs, *d_sreward, *d_sdone, *d_sinfo;
   size_t render_pix; int render_n; int* d_render_ids; unsigned char* d_render_rgba; float* d_render_depth; void* d_render_dev;
-  float *h_dpin_in, *h_dpin_out, *d_daction, *d_dobs, *d_dreward, *d_ddone, *d_dinfo;
-  // CUDA-graph replay of the fused env step (one graph per entry point, keyed by its device pointers)
-  bool use_graph; int graph_failures;
-  struct StepGraph { void* exec; const void* key[5]; uint64_t launches; bool valid; } graphs[4];
   // profiling
   bool profiling;
   std::vector<std::string> knames;
@@ -157,7 +168,6 @@ struct AgSim {
 #define CKP(x) do { cudaError_t err__ = (x); if (err__ != cudaSuccess) { g_err = std::string(#x) + ": " + cudaGetErrorString(err__); return nullptr; } } while (0)
 #endif
 
-extern "C" { static void drop_graph(AgSim* s, int which); }
 static void* dev_alloc(AgSim* s, size_t bytes) {
   void* p = nullptr;
   if (bytes == 0) bytes = 16;
@@ -199,6 +209,38 @@ static int dev_zero(AgSim* s, void* d, size_t bytes) {
 #endif
   return 0;
 }
+// a copy enqueued on the sim's stream; unlike h2d / d2h it does not wait for it
+static int copy_async(AgSim* s, void* dst, const void* src, size_t bytes, cudaMemcpyKind kind) {
+#ifndef AG_CPU_EMU
+  CK(cudaMemcpyAsync(dst, src, bytes, kind, s->stream));
+#else
+  (void)s; (void)kind; memcpy(dst, src, bytes);
+#endif
+  return 0;
+}
+static int pinned_alloc(float** p, size_t floats) {
+#ifndef AG_CPU_EMU
+  CK(cudaMallocHost((void**)p, sizeof(float) * floats));
+#else
+  if (!(*p = (float*)malloc(sizeof(float) * floats))) return fail("host allocation failed");
+#endif
+  return 0;
+}
+static void pinned_free(float* p) {
+#ifndef AG_CPU_EMU
+  if (p) cudaFreeHost(p);
+#else
+  free(p);
+#endif
+}
+static void drop_graph(StepGraph& G) {
+#ifndef AG_CPU_EMU
+  if (G.valid) cudaGraphExecDestroy((cudaGraphExec_t)G.exec);
+#endif
+  G.valid = false;
+}
+// a change to state the fused steps share (a SimDev / ClothDev field a captured kernel holds by value) makes every captured step stale
+static void drop_graphs(AgSim* s) { for (FusedStep& R : s->fused) drop_graph(R.graph); }
 template <typename T>
 static const T* upload(AgSim* s, const std::vector<T>& v) {
   T* d = (T*)dev_alloc(s, v.size() * sizeof(T));
@@ -299,7 +341,7 @@ AgSim* ag_create(const AgSceneDesc* d, const AgConfig* cfg, int n_envs, int devi
   AgSim* s = new AgSim();
   memset(&s->S, 0, sizeof(SimDev));
   memset(&s->F, 0, sizeof(FeedDev));
-  s->cfg = *cfg; s->device = device; s->launches = 0; s->feeding = false; s->bathing = false; s->cloth = false; s->cloth_sub = 0; s->C_dev = nullptr; s->dressing = false; s->DP_dev = nullptr; s->scratch = false; s->SD_dev = nullptr; s->graphs[3].valid = false; s->render_pix = 0; s->render_n = 0; s->d_render_ids = nullptr; s->d_render_rgba = nullptr; s->d_render_depth = nullptr; s->d_render_dev = nullptr; s->graphs[2].valid = false; s->use_graph = true; s->graph_failures = 0; s->graphs[0].valid = s->graphs[1].valid = false; s->B_dev = nullptr; s->stream = nullptr; s->F_dev = nullptr; s->profiling = false;
+  s->cfg = *cfg; s->device = device; s->launches = 0; s->cloth = false; s->cloth_sub = 0; s->C_dev = nullptr; s->DP_dev = nullptr; s->SD_dev = nullptr; s->render_pix = 0; s->render_n = 0; s->d_render_ids = nullptr; s->d_render_rgba = nullptr; s->d_render_depth = nullptr; s->d_render_dev = nullptr; s->use_graph = true; s->graph_failures = 0; s->B_dev = nullptr; s->stream = nullptr; s->F_dev = nullptr; s->profiling = false;
   s->d_stage = nullptr; s->stage_floats = 0;
 #ifndef AG_CPU_EMU
   { int ndev = 0; if (cudaGetDeviceCount(&ndev) != cudaSuccess || device < 0 || device >= ndev) { g_err = "no such CUDA device (is a CUDA device present? there is no CPU fallback)"; delete s; return nullptr; } }
@@ -543,19 +585,11 @@ void ag_destroy(AgSim* s) {
 #ifndef AG_CPU_EMU
   if (s->stream) cudaStreamSynchronize(s->stream);
   for (void* p : s->allocs) cudaFree(p);
-  if (s->feeding) { cudaFreeHost(s->h_pin_in); cudaFreeHost(s->h_pin_out); }
-  if (s->bathing) { cudaFreeHost(s->h_bpin_in); cudaFreeHost(s->h_bpin_out); }
-  if (s->dressing) { cudaFreeHost(s->h_dpin_in); cudaFreeHost(s->h_dpin_out); }
-  if (s->scratch) { cudaFreeHost(s->h_spin_in); cudaFreeHost(s->h_spin_out); }
-  for (int g = 0; g < 4; g++) if (s->graphs[g].valid) cudaGraphExecDestroy((cudaGraphExec_t)s->graphs[g].exec);
   if (s->stream) cudaStreamDestroy(s->stream);
 #else
   for (void* p : s->allocs) free(p);
-  if (s->feeding) { free(s->h_pin_in); free(s->h_pin_out); }
-  if (s->bathing) { free(s->h_bpin_in); free(s->h_bpin_out); }
-  if (s->dressing) { free(s->h_dpin_in); free(s->h_dpin_out); }
-  if (s->scratch) { free(s->h_spin_in); free(s->h_spin_out); }
 #endif
+  for (FusedStep& R : s->fused) { pinned_free(R.h_in); pinned_free(R.h_out); drop_graph(R.graph); }
   delete s;
 }
 
@@ -725,7 +759,7 @@ int ag_set_motor_force_scale(AgSim* s, int n, const int32_t* links, const float*
     if (!s->S.motor_fscale) return fail("device allocation failed");
     std::vector<float> ones(cnt, 1.0f);
     if (h2d(s, s->S.motor_fscale, ones.data(), cnt * sizeof(float))) return -1;
-    for (int g = 0; g < 4; g++) drop_graph(s, g);        // captured kernels hold the SimDev of before (null pointer)
+    drop_graphs(s);                                       // captured kernels hold the SimDev of before (null pointer)
   }
   return scatter_host(s, s->S.motor_fscale, 1, n, links, scale, nullptr);
 }
@@ -980,33 +1014,27 @@ int ag_overflow_count(AgSim* s) {
   return n;
 }
 
-// ------------------------------------------------------------------ CUDA-graph replay of a fused env step
+// ------------------------------------------------------------------ fused env steps: the driver the four tasks share
+// Each task's init fills its FusedStep (fused_alloc) and its enqueue function launches the task's kernels; stepping,
+// graph replay and the host-buffer staging are the same for every task.
+//
 // One env step is ~90 small launches (14 kernels + 3 memsets per substep); captured once per set of device
 // pointers and replayed with a single cudaGraphLaunch.  Falls back to direct launches while profiling
 // (per-kernel events), when AG_GRAPH=0, or if capture fails.
-typedef int (*StepEnqueue)(AgSim*, const float*, float*, float*, float*, float*);
-static void drop_graph(AgSim* s, int which) {
-#ifndef AG_CPU_EMU
-  if (s->graphs[which].valid) { cudaGraphExecDestroy((cudaGraphExec_t)s->graphs[which].exec); s->graphs[which].valid = false; }
-#else
-  (void)s; (void)which;
-#endif
-}
-static int run_step(AgSim* s, int which, StepEnqueue enq, const float* action, float* obs, float* reward, float* done, float* info) {
+static int run_step(AgSim* s, FusedStep& R, const float* action, float* obs, float* reward, float* done, float* info) {
 #ifndef AG_CPU_EMU
   if (s->use_graph && !s->profiling) {
-    // The graph is captured against the sim's OWN action buffer: a learner hands in a freshly allocated action tensor
+    // The graph is captured against the task's OWN action buffer: a learner hands in a freshly allocated action tensor
     // every step, and a graph keyed on that address would be re-captured (~90 launches + instantiate) each time.
-    float* own = which == 0 ? s->d_action : (which == 1 ? s->d_baction : (which == 2 ? s->d_daction : s->d_saction));
-    if (action != own) { CK(cudaMemcpyAsync(own, action, sizeof(float) * 7 * s->S.N, cudaMemcpyDeviceToDevice, s->stream)); action = own; }
-    AgSim::StepGraph& G = s->graphs[which];
+    if (action != R.d_action) { CK(cudaMemcpyAsync(R.d_action, action, sizeof(float) * 7 * s->S.N, cudaMemcpyDeviceToDevice, s->stream)); action = R.d_action; }
+    StepGraph& G = R.graph;
     const void* key[5] = {action, obs, reward, done, info};
-    if (G.valid && memcmp(G.key, key, sizeof(key)) != 0) { cudaGraphExecDestroy((cudaGraphExec_t)G.exec); G.valid = false; }
+    if (G.valid && memcmp(G.key, key, sizeof(key)) != 0) drop_graph(G);
     if (!G.valid) {
       uint64_t l0 = s->launches;
       cudaGraph_t graph = nullptr; cudaGraphExec_t exec = nullptr;
       if (cudaStreamBeginCapture(s->stream, cudaStreamCaptureModeThreadLocal) == cudaSuccess) {
-        int rc = enq(s, action, obs, reward, done, info);
+        int rc = R.enqueue(s, action, obs, reward, done, info);
         cudaError_t ce = cudaStreamEndCapture(s->stream, &graph);
         if (rc == 0 && ce == cudaSuccess && graph && cudaGraphInstantiate(&exec, graph, 0) == cudaSuccess) {
           G.exec = exec; memcpy(G.key, key, sizeof(key)); G.launches = s->launches - l0; G.valid = true; s->graph_failures = 0;
@@ -1022,10 +1050,82 @@ static int run_step(AgSim* s, int which, StepEnqueue enq, const float* action, f
       return 0;
     }
   }
-#else
-  (void)which;
 #endif
-  return enq(s, action, obs, reward, done, info);
+  return R.enqueue(s, action, obs, reward, done, info);
+}
+// Allocates task t's step I/O on its first init; a later init (an episode reset) keeps the buffers.
+static int fused_alloc(AgSim* s, FusedTask t, int obs_dim, StepEnqueue enqueue) {
+  FusedStep& R = s->fused[t];
+  R.obs_dim = obs_dim; R.enqueue = enqueue;
+  if (R.h_out) return 0;
+  const size_t N = s->S.N;
+  R.d_action = dalloc<float>(s, N * 7); R.d_obs = dalloc<float>(s, N * obs_dim);
+  R.d_reward = dalloc<float>(s, N); R.d_done = dalloc<float>(s, N); R.d_info = dalloc<float>(s, N * 4);
+  if (!R.d_action || !R.d_obs || !R.d_reward || !R.d_done || !R.d_info) return fail("device allocation failed");
+  if (!R.h_in && pinned_alloc(&R.h_in, N * 7)) return -1;
+  return pinned_alloc(&R.h_out, N * (obs_dim + 6));
+}
+static int need_init(AgSim* s, FusedTask t) {
+  return s->fused[t].ready ? 0 : fail(std::string("ag_") + fused_name[t] + "_init not called");
+}
+// device-buffer step: enqueued on the sim's stream, returns without waiting for it
+static int fused_step_dev(AgSim* s, FusedTask t, const float* action, float* obs, float* reward, float* done, float* info) {
+  if (need_init(s, t)) return -1;
+  if (s->cloth && s->cloth_sub != 0)
+    return fail(std::string("ag_") + fused_name[t] + "_step: a stepSimulation is half done (ag_step with a partial substep count?)");
+  int rc = run_step(s, s->fused[t], action, obs, reward, done, info);
+#ifndef AG_CPU_EMU
+  CK(cudaGetLastError());
+#endif
+  return rc;
+}
+// host-buffer step in two halves: `begin` stages the actions (pinned) and enqueues H2D, the fused step and the D2H
+// read-back on the sim's stream and returns; `end` waits for that stream and hands the results out (`info` may be NULL).
+// Several sims (sub-batches of one batch, each on its own stream) overlap this way.
+static int fused_step_host_begin(AgSim* s, FusedTask t, const float* action) {
+  if (need_init(s, t)) return -1;
+  FusedStep& R = s->fused[t];
+  const size_t N = s->S.N, D = R.obs_dim;
+  float* o = R.h_out;
+  memcpy(R.h_in, action, sizeof(float) * N * 7);
+  if (copy_async(s, R.d_action, R.h_in, sizeof(float) * N * 7, cudaMemcpyHostToDevice)) return -1;
+  if (fused_step_dev(s, t, R.d_action, R.d_obs, R.d_reward, R.d_done, R.d_info)) return -1;
+  if (copy_async(s, o, R.d_obs, sizeof(float) * N * D, cudaMemcpyDeviceToHost) ||
+      copy_async(s, o + N * D, R.d_reward, sizeof(float) * N, cudaMemcpyDeviceToHost) ||
+      copy_async(s, o + N * (D + 1), R.d_done, sizeof(float) * N, cudaMemcpyDeviceToHost) ||
+      copy_async(s, o + N * (D + 2), R.d_info, sizeof(float) * N * 4, cudaMemcpyDeviceToHost)) return -1;
+  return 0;
+}
+static int fused_step_host_end(AgSim* s, FusedTask t, float* obs, float* reward, float* done, float* info) {
+  if (need_init(s, t)) return -1;
+  const FusedStep& R = s->fused[t];
+  const size_t N = s->S.N, D = R.obs_dim;
+#ifndef AG_CPU_EMU
+  CK(cudaStreamSynchronize(s->stream));
+  CK(cudaGetLastError());
+#endif
+  memcpy(obs, R.h_out, sizeof(float) * N * D);
+  memcpy(reward, R.h_out + N * D, sizeof(float) * N);
+  memcpy(done, R.h_out + N * (D + 1), sizeof(float) * N);
+  if (info) memcpy(info, R.h_out + N * (D + 2), sizeof(float) * N * 4);
+  return 0;
+}
+static int fused_step_host(AgSim* s, FusedTask t, const float* action, float* obs, float* reward, float* done, float* info) {
+  if (fused_step_host_begin(s, t, action)) return -1;
+  return fused_step_host_end(s, t, obs, reward, done, info);
+}
+// tremor of `nj` joints of the person: per env on/off, rest angles and amplitudes [N][nj] -> the task's [N], [nj][N], [nj][N]
+// device arrays.  NULL `on` switches tremor off.
+static int set_tremor(AgSim* s, FusedTask t, int nj, int* d_on, float* d_rest, float* d_amp, const int32_t* on, const float* rest, const float* amplitude) {
+  if (need_init(s, t)) return -1;
+  const int N = s->S.N;
+  std::vector<int> o(N, 0); std::vector<float> r((size_t)nj * N, 0.f), a((size_t)nj * N, 0.f);
+  if (on) for (int e = 0; e < N; e++) {
+    o[e] = on[e];
+    for (int j = 0; j < nj; j++) { r[(size_t)j * N + e] = rest ? rest[(size_t)e * nj + j] : 0.f; a[(size_t)j * N + e] = amplitude ? amplitude[(size_t)e * nj + j] : 0.f; }
+  }
+  if (h2d(s, d_on, o.data(), sizeof(int) * N) || h2d(s, d_rest, r.data(), sizeof(float) * nj * N)) return -1;
+  return h2d(s, d_amp, a.data(), sizeof(float) * nj * N);
 }
 
 // ------------------------------------------------------------------ cloth (K8, ag_cloth.cuh)
@@ -1132,7 +1232,7 @@ int ag_cloth_init(AgSim* s, const AgClothDesc* d) {
   if (s->cloth_npt == 4) { CK(cudaFuncSetAttribute(k_cloth<4, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024)); CK(cudaFuncSetAttribute(k_cloth<4, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024)); }
   else { CK(cudaFuncSetAttribute(k_cloth<8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024)); CK(cudaFuncSetAttribute(k_cloth<8, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024)); }
 #endif
-  drop_graph(s, 0); drop_graph(s, 1); drop_graph(s, 2);
+  drop_graphs(s);                                     // a captured step has no cloth launch
   s->cloth = true; s->cloth_sub = 0;
   return 0;
 }
@@ -1188,7 +1288,7 @@ int ag_cloth_set_gravity(AgSim* s, const double g[3]) {
   DevGuard guard__(s->device);
   if (!s->cloth) return fail("ag_cloth_init not called");
   s->C.gx = (float)g[0]; s->C.gy = (float)g[1]; s->C.gz = (float)g[2];
-  drop_graph(s, 0); drop_graph(s, 1); drop_graph(s, 2);   // k_cloth takes ClothDev by value: a captured step holds the old gravity
+  drop_graphs(s);                                       // k_cloth takes ClothDev by value: a captured step holds the old gravity
   return cloth_refresh(s);
 }
 int ag_cloth_get_contacts(AgSim* s, int max_pts, int32_t* count, int32_t* node, float* pos, float* force, int32_t* link) {
@@ -1221,57 +1321,13 @@ int ag_cloth_device_state(AgSim* s, float** x_dev, float** v_dev, int32_t* nnp) 
 // ------------------------------------------------------------------ fused DressingEnv path
 int ag_dressing_reset_episode(AgSim* s, const int32_t* env_mask) {
   DevGuard guard__(s->device);
-  if (!s->dressing) return fail("ag_dressing_init not called");
+  if (need_init(s, FT_DRESSING)) return -1;
   const int N = s->S.N;
   std::vector<int> it(N); std::vector<float> ts(N);
   if (d2h(s, it.data(), s->DP.D.iteration, sizeof(int) * N) || d2h(s, ts.data(), s->DP.D.task_success, sizeof(float) * N)) return -1;
   for (int e = 0; e < N; e++) if (!env_mask || env_mask[e]) { it[e] = 0; ts[e] = 0.f; }
   if (h2d(s, s->DP.D.iteration, it.data(), sizeof(int) * N) || h2d(s, s->DP.D.task_success, ts.data(), sizeof(float) * N)) return -1;
   return 0;
-}
-int ag_dressing_init(AgSim* s, const AgDressingParams* p, const int32_t* gender_is_male) {
-  DevGuard guard__(s->device);
-  if (!s->cloth) return fail("ag_dressing_init: ag_cloth_init first");
-  const int N = s->S.N;
-  for (int j = 0; j < 7; j++) if (p->arm_links[j] < 0 || p->arm_links[j] >= s->nl) return fail("ag_dressing_init: bad arm link");
-  for (int j = 0; j < 3; j++) if (p->tri1[j] < 0 || p->tri1[j] >= s->C.nn || p->tri2[j] < 0 || p->tri2[j] >= s->C.nn) return fail("ag_dressing_init: bad sleeve node");
-  if (p->ee_link < 0 || p->ee_link >= s->nl) return fail("ag_dressing_init: bad end effector link");
-  DressDev& D = s->DP.D;
-  D.P = *p;
-  drop_graph(s, 2);
-  if (!s->dressing) {
-    D.male = dalloc<int>(s, N); D.iteration = dalloc<int>(s, N); D.task_success = dalloc<float>(s, N); D.action = dalloc<float>(s, (size_t)N * 7);
-    D.tremor_on = dalloc<int>(s, N); D.tremor_rest = dalloc<float>(s, (size_t)N * 10); D.tremor_amp = dalloc<float>(s, (size_t)N * 10);
-    s->d_daction = dalloc<float>(s, (size_t)N * 7); s->d_dobs = dalloc<float>(s, (size_t)N * 24);
-    s->d_dreward = dalloc<float>(s, N); s->d_ddone = dalloc<float>(s, N); s->d_dinfo = dalloc<float>(s, (size_t)N * 4);
-    s->DP_dev = dalloc<DressPost>(s, 1);
-    if (!s->d_dinfo || !s->DP_dev) return fail("device allocation failed");
-#ifndef AG_CPU_EMU
-    CK(cudaMallocHost((void**)&s->h_dpin_in, sizeof(float) * N * 7));
-    CK(cudaMallocHost((void**)&s->h_dpin_out, sizeof(float) * N * 30));
-#else
-    s->h_dpin_in = (float*)malloc(sizeof(float) * N * 7); s->h_dpin_out = (float*)malloc(sizeof(float) * N * 30);
-#endif
-  }
-  else if (dev_zero(s, D.tremor_on, sizeof(int) * N)) return -1;
-  for (int j = 0; j < 10; j++) if (p->human_arm_m[j] < 0 || p->human_arm_m[j] >= s->nl || p->human_arm_f[j] < 0 || p->human_arm_f[j] >= s->nl) return fail("ag_dressing_init: bad human arm link");
-  s->DP.C = s->C_dev;
-  if (h2d(s, D.male, gender_is_male, sizeof(int) * N)) return -1;
-  if (h2d(s, s->DP_dev, &s->DP, sizeof(DressPost))) return -1;
-  s->dressing = true;
-  return ag_dressing_reset_episode(s, nullptr);
-}
-int ag_dressing_set_tremor(AgSim* s, const int32_t* on, const float* rest, const float* amplitude) {
-  DevGuard guard__(s->device);
-  if (!s->dressing) return fail("ag_dressing_init not called");
-  const int N = s->S.N;
-  std::vector<int> o(N, 0); std::vector<float> r((size_t)10 * N, 0.f), a((size_t)10 * N, 0.f);
-  if (on) for (int e = 0; e < N; e++) {
-    o[e] = on[e];
-    for (int j = 0; j < 10; j++) { r[(size_t)j * N + e] = rest ? rest[(size_t)e * 10 + j] : 0.f; a[(size_t)j * N + e] = amplitude ? amplitude[(size_t)e * 10 + j] : 0.f; }
-  }
-  if (h2d(s, s->DP.D.tremor_on, o.data(), sizeof(int) * N) || h2d(s, s->DP.D.tremor_rest, r.data(), sizeof(float) * 10 * N)) return -1;
-  return h2d(s, s->DP.D.tremor_amp, a.data(), sizeof(float) * 10 * N);
 }
 static int dressing_step_enqueue(AgSim* s, const float* action_dev, float* obs, float* reward, float* done, float* info) {
   const int N = s->S.N;
@@ -1289,42 +1345,39 @@ static int dressing_step_enqueue(AgSim* s, const float* action_dev, float* obs, 
   LAUNCH(s, k_dress_post, N, q);
   return 0;
 }
-int ag_dressing_step_dev(AgSim* s, const float* action_dev, float* obs_dev, float* reward_dev, float* done_dev, float* info_dev) {
+int ag_dressing_init(AgSim* s, const AgDressingParams* p, const int32_t* gender_is_male) {
   DevGuard guard__(s->device);
-  if (!s->dressing) return fail("ag_dressing_init not called");
-  if (s->cloth_sub != 0) return fail("ag_dressing_step: a stepSimulation is half done (ag_step with a partial substep count?)");
-  int rc = run_step(s, 2, dressing_step_enqueue, action_dev, obs_dev, reward_dev, done_dev, info_dev);
-#ifndef AG_CPU_EMU
-  CK(cudaGetLastError());
-#endif
-  return rc;
-}
-int ag_dressing_step_host(AgSim* s, const float* action, float* obs, float* reward, float* done, float* info) {
-  DevGuard guard__(s->device);
-  if (!s->dressing) return fail("ag_dressing_init not called");
+  if (!s->cloth) return fail("ag_dressing_init: ag_cloth_init first");
   const int N = s->S.N;
-  memcpy(s->h_dpin_in, action, sizeof(float) * N * 7);
-#ifndef AG_CPU_EMU
-  CK(cudaMemcpyAsync(s->d_daction, s->h_dpin_in, sizeof(float) * N * 7, cudaMemcpyHostToDevice, s->stream));
-#else
-  memcpy(s->d_daction, s->h_dpin_in, sizeof(float) * N * 7);
-#endif
-  if (ag_dressing_step_dev(s, s->d_daction, s->d_dobs, s->d_dreward, s->d_ddone, s->d_dinfo)) return -1;
-  float* o = s->h_dpin_out;
-#ifndef AG_CPU_EMU
-  CK(cudaMemcpyAsync(o, s->d_dobs, sizeof(float) * N * 24, cudaMemcpyDeviceToHost, s->stream));
-  CK(cudaMemcpyAsync(o + (size_t)N * 24, s->d_dreward, sizeof(float) * N, cudaMemcpyDeviceToHost, s->stream));
-  CK(cudaMemcpyAsync(o + (size_t)N * 25, s->d_ddone, sizeof(float) * N, cudaMemcpyDeviceToHost, s->stream));
-  CK(cudaMemcpyAsync(o + (size_t)N * 26, s->d_dinfo, sizeof(float) * N * 4, cudaMemcpyDeviceToHost, s->stream));
-  CK(cudaStreamSynchronize(s->stream));
-#else
-  memcpy(o, s->d_dobs, sizeof(float) * N * 24); memcpy(o + (size_t)N * 24, s->d_dreward, sizeof(float) * N);
-  memcpy(o + (size_t)N * 25, s->d_ddone, sizeof(float) * N); memcpy(o + (size_t)N * 26, s->d_dinfo, sizeof(float) * N * 4);
-#endif
-  memcpy(obs, o, sizeof(float) * N * 24); memcpy(reward, o + (size_t)N * 24, sizeof(float) * N);
-  memcpy(done, o + (size_t)N * 25, sizeof(float) * N); memcpy(info, o + (size_t)N * 26, sizeof(float) * N * 4);
-  return 0;
+  for (int j = 0; j < 7; j++) if (p->arm_links[j] < 0 || p->arm_links[j] >= s->nl) return fail("ag_dressing_init: bad arm link");
+  for (int j = 0; j < 3; j++) if (p->tri1[j] < 0 || p->tri1[j] >= s->C.nn || p->tri2[j] < 0 || p->tri2[j] >= s->C.nn) return fail("ag_dressing_init: bad sleeve node");
+  if (p->ee_link < 0 || p->ee_link >= s->nl) return fail("ag_dressing_init: bad end effector link");
+  DressDev& D = s->DP.D;
+  D.P = *p;
+  drop_graph(s->fused[FT_DRESSING].graph);
+  if (!s->fused[FT_DRESSING].ready) {
+    D.male = dalloc<int>(s, N); D.iteration = dalloc<int>(s, N); D.task_success = dalloc<float>(s, N); D.action = dalloc<float>(s, (size_t)N * 7);
+    D.tremor_on = dalloc<int>(s, N); D.tremor_rest = dalloc<float>(s, (size_t)N * 10); D.tremor_amp = dalloc<float>(s, (size_t)N * 10);
+    s->DP_dev = dalloc<DressPost>(s, 1);
+    if (!s->DP_dev) return fail("device allocation failed");
+  }
+  else if (dev_zero(s, D.tremor_on, sizeof(int) * N)) return -1;
+  if (fused_alloc(s, FT_DRESSING, 24, dressing_step_enqueue)) return -1;
+  for (int j = 0; j < 10; j++) if (p->human_arm_m[j] < 0 || p->human_arm_m[j] >= s->nl || p->human_arm_f[j] < 0 || p->human_arm_f[j] >= s->nl) return fail("ag_dressing_init: bad human arm link");
+  s->DP.C = s->C_dev;
+  if (h2d(s, D.male, gender_is_male, sizeof(int) * N)) return -1;
+  if (h2d(s, s->DP_dev, &s->DP, sizeof(DressPost))) return -1;
+  s->fused[FT_DRESSING].ready = true;
+  return ag_dressing_reset_episode(s, nullptr);
 }
+int ag_dressing_set_tremor(AgSim* s, const int32_t* on, const float* rest, const float* amplitude) {
+  DevGuard guard__(s->device);
+  return set_tremor(s, FT_DRESSING, 10, s->DP.D.tremor_on, s->DP.D.tremor_rest, s->DP.D.tremor_amp, on, rest, amplitude);
+}
+int ag_dressing_step_dev(AgSim* s, const float* action_dev, float* obs_dev, float* reward_dev, float* done_dev, float* info_dev) {
+  DevGuard guard__(s->device); return fused_step_dev(s, FT_DRESSING, action_dev, obs_dev, reward_dev, done_dev, info_dev); }
+int ag_dressing_step_host(AgSim* s, const float* action, float* obs, float* reward, float* done, float* info) {
+  DevGuard guard__(s->device); return fused_step_host(s, FT_DRESSING, action, obs, reward, done, info); }
 
 // ------------------------------------------------------------------ camera images (K9, ag_render.cuh)
 int ag_render(AgSim* s, const AgCamera* cam, int n, const int32_t* env_ids, uint8_t* rgba, float* depth) {
@@ -1363,37 +1416,6 @@ int ag_render(AgSim* s, const AgCamera* cam, int n, const int32_t* env_ids, uint
 }
 
 // ------------------------------------------------------------------ fused ScratchItchEnv path
-int ag_scratch_init(AgSim* s, const AgScratchParams* p, const int32_t* gender_is_male, const int32_t* limb_link, const float* target_local) {
-  DevGuard guard__(s->device);
-  const int N = s->S.N;
-  for (int j = 0; j < 7; j++) if (p->arm_links[j] < 0 || p->arm_links[j] >= s->nl) return fail("ag_scratch_init: bad arm link");
-  if (p->ee_link < 0 || p->ee_link >= s->nl || p->tool_tip_link < 0 || p->tool_tip_link >= s->nl || p->tool_link0 < 0 || p->tool_link0 >= s->nl) return fail("ag_scratch_init: bad link");
-  for (int e = 0; e < N; e++) if (limb_link[e] < 0 || limb_link[e] >= s->nl) return fail("ag_scratch_init: bad limb link");
-  ScratchDev& D = s->SD;
-  D.P = *p;
-  drop_graph(s, 3);
-  if (!s->scratch) {
-    D.male = dalloc<int>(s, N); D.iteration = dalloc<int>(s, N); D.task_success = dalloc<int>(s, N); D.limb_link = dalloc<int>(s, N);
-    D.target_local = dalloc<float>(s, (size_t)3 * N); D.prev_contact = dalloc<float>(s, (size_t)3 * N); D.action = dalloc<float>(s, (size_t)7 * N);
-    s->d_saction = dalloc<float>(s, (size_t)N * 7); s->d_sobs = dalloc<float>(s, (size_t)N * 30);
-    s->d_sreward = dalloc<float>(s, N); s->d_sdone = dalloc<float>(s, N); s->d_sinfo = dalloc<float>(s, (size_t)N * 4);
-    s->SD_dev = dalloc<ScratchDev>(s, 1);
-    if (!s->d_sinfo || !s->SD_dev) return fail("device allocation failed");
-#ifndef AG_CPU_EMU
-    CK(cudaMallocHost((void**)&s->h_spin_in, sizeof(float) * N * 7));
-    CK(cudaMallocHost((void**)&s->h_spin_out, sizeof(float) * N * 36));
-#else
-    s->h_spin_in = (float*)malloc(sizeof(float) * N * 7); s->h_spin_out = (float*)malloc(sizeof(float) * N * 36);
-#endif
-  }
-  std::vector<float> tl((size_t)3 * N);
-  for (int e = 0; e < N; e++) for (int c = 0; c < 3; c++) tl[(size_t)c * N + e] = target_local[(size_t)e * 3 + c];
-  if (h2d(s, D.male, gender_is_male, sizeof(int) * N) || h2d(s, D.limb_link, limb_link, sizeof(int) * N) || h2d(s, D.target_local, tl.data(), sizeof(float) * 3 * N)) return -1;
-  if (dev_zero(s, D.iteration, sizeof(int) * N) || dev_zero(s, D.task_success, sizeof(int) * N) || dev_zero(s, D.prev_contact, sizeof(float) * 3 * N)) return -1;   // scratch_itch.py:97
-  if (h2d(s, s->SD_dev, &s->SD, sizeof(ScratchDev))) return -1;
-  s->scratch = true;
-  return 0;
-}
 static int scratch_step_enqueue(AgSim* s, const float* action_dev, float* obs, float* reward, float* done, float* info) {
   const int N = s->S.N;
   KP p = kp0(); p.p0 = action_dev; p.p1 = s->SD_dev;
@@ -1405,104 +1427,36 @@ static int scratch_step_enqueue(AgSim* s, const float* action_dev, float* obs, f
   LAUNCH(s, k_scratch_post, N, q);
   return 0;
 }
-int ag_scratch_step_dev(AgSim* s, const float* action_dev, float* obs_dev, float* reward_dev, float* done_dev, float* info_dev) {
+int ag_scratch_init(AgSim* s, const AgScratchParams* p, const int32_t* gender_is_male, const int32_t* limb_link, const float* target_local) {
   DevGuard guard__(s->device);
-  if (!s->scratch) return fail("ag_scratch_init not called");
-  int rc = run_step(s, 3, scratch_step_enqueue, action_dev, obs_dev, reward_dev, done_dev, info_dev);
-#ifndef AG_CPU_EMU
-  CK(cudaGetLastError());
-#endif
-  return rc;
-}
-int ag_scratch_step_host(AgSim* s, const float* action, float* obs, float* reward, float* done, float* info) {
-  DevGuard guard__(s->device);
-  if (!s->scratch) return fail("ag_scratch_init not called");
   const int N = s->S.N;
-  memcpy(s->h_spin_in, action, sizeof(float) * N * 7);
-#ifndef AG_CPU_EMU
-  CK(cudaMemcpyAsync(s->d_saction, s->h_spin_in, sizeof(float) * N * 7, cudaMemcpyHostToDevice, s->stream));
-#else
-  memcpy(s->d_saction, s->h_spin_in, sizeof(float) * N * 7);
-#endif
-  if (ag_scratch_step_dev(s, s->d_saction, s->d_sobs, s->d_sreward, s->d_sdone, s->d_sinfo)) return -1;
-  float* o = s->h_spin_out;
-#ifndef AG_CPU_EMU
-  CK(cudaMemcpyAsync(o, s->d_sobs, sizeof(float) * N * 30, cudaMemcpyDeviceToHost, s->stream));
-  CK(cudaMemcpyAsync(o + (size_t)N * 30, s->d_sreward, sizeof(float) * N, cudaMemcpyDeviceToHost, s->stream));
-  CK(cudaMemcpyAsync(o + (size_t)N * 31, s->d_sdone, sizeof(float) * N, cudaMemcpyDeviceToHost, s->stream));
-  CK(cudaMemcpyAsync(o + (size_t)N * 32, s->d_sinfo, sizeof(float) * N * 4, cudaMemcpyDeviceToHost, s->stream));
-  CK(cudaStreamSynchronize(s->stream));
-#else
-  memcpy(o, s->d_sobs, sizeof(float) * N * 30); memcpy(o + (size_t)N * 30, s->d_sreward, sizeof(float) * N);
-  memcpy(o + (size_t)N * 31, s->d_sdone, sizeof(float) * N); memcpy(o + (size_t)N * 32, s->d_sinfo, sizeof(float) * N * 4);
-#endif
-  memcpy(obs, o, sizeof(float) * N * 30); memcpy(reward, o + (size_t)N * 30, sizeof(float) * N);
-  memcpy(done, o + (size_t)N * 31, sizeof(float) * N); memcpy(info, o + (size_t)N * 32, sizeof(float) * N * 4);
+  for (int j = 0; j < 7; j++) if (p->arm_links[j] < 0 || p->arm_links[j] >= s->nl) return fail("ag_scratch_init: bad arm link");
+  if (p->ee_link < 0 || p->ee_link >= s->nl || p->tool_tip_link < 0 || p->tool_tip_link >= s->nl || p->tool_link0 < 0 || p->tool_link0 >= s->nl) return fail("ag_scratch_init: bad link");
+  for (int e = 0; e < N; e++) if (limb_link[e] < 0 || limb_link[e] >= s->nl) return fail("ag_scratch_init: bad limb link");
+  ScratchDev& D = s->SD;
+  D.P = *p;
+  drop_graph(s->fused[FT_SCRATCH].graph);
+  if (!s->fused[FT_SCRATCH].ready) {
+    D.male = dalloc<int>(s, N); D.iteration = dalloc<int>(s, N); D.task_success = dalloc<int>(s, N); D.limb_link = dalloc<int>(s, N);
+    D.target_local = dalloc<float>(s, (size_t)3 * N); D.prev_contact = dalloc<float>(s, (size_t)3 * N); D.action = dalloc<float>(s, (size_t)7 * N);
+    s->SD_dev = dalloc<ScratchDev>(s, 1);
+    if (!s->SD_dev) return fail("device allocation failed");
+  }
+  if (fused_alloc(s, FT_SCRATCH, 30, scratch_step_enqueue)) return -1;
+  std::vector<float> tl((size_t)3 * N);
+  for (int e = 0; e < N; e++) for (int c = 0; c < 3; c++) tl[(size_t)c * N + e] = target_local[(size_t)e * 3 + c];
+  if (h2d(s, D.male, gender_is_male, sizeof(int) * N) || h2d(s, D.limb_link, limb_link, sizeof(int) * N) || h2d(s, D.target_local, tl.data(), sizeof(float) * 3 * N)) return -1;
+  if (dev_zero(s, D.iteration, sizeof(int) * N) || dev_zero(s, D.task_success, sizeof(int) * N) || dev_zero(s, D.prev_contact, sizeof(float) * 3 * N)) return -1;   // scratch_itch.py:97
+  if (h2d(s, s->SD_dev, &s->SD, sizeof(ScratchDev))) return -1;
+  s->fused[FT_SCRATCH].ready = true;
   return 0;
 }
+int ag_scratch_step_dev(AgSim* s, const float* action_dev, float* obs_dev, float* reward_dev, float* done_dev, float* info_dev) {
+  DevGuard guard__(s->device); return fused_step_dev(s, FT_SCRATCH, action_dev, obs_dev, reward_dev, done_dev, info_dev); }
+int ag_scratch_step_host(AgSim* s, const float* action, float* obs, float* reward, float* done, float* info) {
+  DevGuard guard__(s->device); return fused_step_host(s, FT_SCRATCH, action, obs, reward, done, info); }
 
 // ------------------------------------------------------------------ fused FeedingEnv path
-int ag_feeding_init(AgSim* s, const AgFeedingParams* p, const int32_t* gender_is_male) {
-  DevGuard guard__(s->device);
-  const int N = s->S.N;
-  FeedDev& F = s->F;
-  F.P = *p;
-  if (p->n_foods > 16) return fail("too many foods");
-  drop_graph(s, 0);           // the captured step refers to the previous FeedDev
-  if (!s->feeding) {          // buffers are allocated once; a later init (episode reset) only refreshes their contents
-    F.male = dalloc<int>(s, N); F.food_state = dalloc<int>(s, N); F.iteration = dalloc<int>(s, N); F.task_success = dalloc<int>(s, N);
-    F.food_near = dalloc<int>(s, (size_t)N * 16);
-    F.action = dalloc<float>(s, (size_t)N * 7); F.rng = dalloc<unsigned long long>(s, N);
-    F.tremor_on = dalloc<int>(s, N); F.tremor_rest = dalloc<float>(s, (size_t)N * 4); F.tremor_amp = dalloc<float>(s, (size_t)N * 4);
-    s->d_action = dalloc<float>(s, (size_t)N * 7); s->d_obs = dalloc<float>(s, (size_t)N * 25);
-    s->d_reward = dalloc<float>(s, N); s->d_done = dalloc<float>(s, N); s->d_info = dalloc<float>(s, (size_t)N * 4);
-    s->F_dev = dalloc<FeedDev>(s, 1);
-    if (!s->d_info || !s->F_dev) return fail("device allocation failed");
-#ifndef AG_CPU_EMU
-    CK(cudaMallocHost((void**)&s->h_pin_in, sizeof(float) * N * 7));
-    CK(cudaMallocHost((void**)&s->h_pin_out, sizeof(float) * N * 31));
-#else
-    s->h_pin_in = (float*)malloc(sizeof(float) * N * 7); s->h_pin_out = (float*)malloc(sizeof(float) * N * 31);
-#endif
-  } else {
-    if (dev_zero(s, F.tremor_on, sizeof(int) * N) || dev_zero(s, F.rng, sizeof(unsigned long long) * N)) return -1;
-  }
-  if (h2d(s, F.male, gender_is_male, sizeof(int) * N)) return -1;
-  if (!s->F_dev || h2d(s, s->F_dev, &s->F, sizeof(FeedDev))) return fail("FeedDev upload failed");
-  s->feeding = true;
-  return ag_feeding_reset_episode(s, nullptr);
-}
-int ag_feeding_set_tremor(AgSim* s, const int32_t* on, const float* rest, const float* amplitude) {
-  DevGuard guard__(s->device);
-  if (!s->feeding) return fail("ag_feeding_init not called");
-  const int N = s->S.N;
-  std::vector<int> o(N, 0); std::vector<float> r((size_t)4 * N, 0.f), a((size_t)4 * N, 0.f);
-  if (on) for (int e = 0; e < N; e++) {
-    o[e] = on[e];
-    for (int j = 0; j < 4; j++) { r[(size_t)j * N + e] = rest ? rest[(size_t)e * 4 + j] : 0.f; a[(size_t)j * N + e] = amplitude ? amplitude[(size_t)e * 4 + j] : 0.f; }
-  }
-  if (h2d(s, s->F.tremor_on, o.data(), sizeof(int) * N)) return -1;
-  if (h2d(s, s->F.tremor_rest, r.data(), sizeof(float) * 4 * N)) return -1;
-  return h2d(s, s->F.tremor_amp, a.data(), sizeof(float) * 4 * N);
-}
-
-int ag_feeding_reset_episode(AgSim* s, const int32_t* env_mask) {
-  DevGuard guard__(s->device);
-  if (!s->feeding) return fail("ag_feeding_init not called");
-  const int N = s->S.N;
-  std::vector<int> fs(N), it(N), ts(N); std::vector<unsigned long long> rng(N);
-  d2h(s, fs.data(), s->F.food_state, sizeof(int) * N); d2h(s, it.data(), s->F.iteration, sizeof(int) * N);
-  d2h(s, ts.data(), s->F.task_success, sizeof(int) * N); d2h(s, rng.data(), s->F.rng, sizeof(unsigned long long) * N);
-  int full = (1 << s->F.P.n_foods) - 1;
-  for (int e = 0; e < N; e++) if (!env_mask || env_mask[e]) {
-    fs[e] = full | (full << 16); it[e] = 0; ts[e] = 0;
-    if (rng[e] == 0) rng[e] = (s->F.P.seed + 0x9E3779B97F4A7C15ull * (unsigned long long)(e + 1)) | 1ull;
-  }
-  h2d(s, s->F.food_state, fs.data(), sizeof(int) * N); h2d(s, s->F.iteration, it.data(), sizeof(int) * N);
-  h2d(s, s->F.task_success, ts.data(), sizeof(int) * N); h2d(s, s->F.rng, rng.data(), sizeof(unsigned long long) * N);
-  return 0;
-}
-
 static int feeding_step_enqueue(AgSim* s, const float* action_dev, float* obs, float* reward, float* done, float* info) {
   const int N = s->S.N;
   KP p = kp0(); p.p0 = action_dev; p.p1 = s->F_dev;
@@ -1520,101 +1474,61 @@ static int feeding_step_enqueue(AgSim* s, const float* action_dev, float* obs, f
   LAUNCH(s, k_feed_post, N, q);
   return 0;
 }
-int ag_feeding_step_dev(AgSim* s, const float* action_dev, float* obs_dev, float* reward_dev, float* done_dev, float* info_dev) {
+int ag_feeding_init(AgSim* s, const AgFeedingParams* p, const int32_t* gender_is_male) {
   DevGuard guard__(s->device);
-  if (!s->feeding) return fail("ag_feeding_init not called");
-  int rc = run_step(s, 0, feeding_step_enqueue, action_dev, obs_dev, reward_dev, done_dev, info_dev);
-#ifndef AG_CPU_EMU
-  CK(cudaGetLastError());
-#endif
-  return rc;
-}
-// host-buffer step in two halves: `begin` stages the actions (pinned) and enqueues H2D, the fused step and the D2H
-// read-back on the sim's stream and returns; `end` waits for that stream and hands the results out.  Several sims
-// (sub-batches of one batch, each on its own stream) overlap this way; ag_feeding_step_host = begin + end.
-int ag_feeding_step_host_begin(AgSim* s, const float* action) {
-  DevGuard guard__(s->device);
-  if (!s->feeding) return fail("ag_feeding_init not called");
   const int N = s->S.N;
-  memcpy(s->h_pin_in, action, sizeof(float) * N * 7);
-#ifndef AG_CPU_EMU
-  CK(cudaMemcpyAsync(s->d_action, s->h_pin_in, sizeof(float) * N * 7, cudaMemcpyHostToDevice, s->stream));
-#else
-  memcpy(s->d_action, s->h_pin_in, sizeof(float) * N * 7);
-#endif
-  if (run_step(s, 0, feeding_step_enqueue, s->d_action, s->d_obs, s->d_reward, s->d_done, s->d_info)) return -1;
-#ifndef AG_CPU_EMU
-  CK(cudaMemcpyAsync(s->h_pin_out, s->d_obs, sizeof(float) * N * 25, cudaMemcpyDeviceToHost, s->stream));
-  CK(cudaMemcpyAsync(s->h_pin_out + (size_t)N * 25, s->d_reward, sizeof(float) * N, cudaMemcpyDeviceToHost, s->stream));
-  CK(cudaMemcpyAsync(s->h_pin_out + (size_t)N * 26, s->d_done, sizeof(float) * N, cudaMemcpyDeviceToHost, s->stream));
-  CK(cudaMemcpyAsync(s->h_pin_out + (size_t)N * 27, s->d_info, sizeof(float) * N * 4, cudaMemcpyDeviceToHost, s->stream));
-#else
-  memcpy(s->h_pin_out, s->d_obs, sizeof(float) * N * 25); memcpy(s->h_pin_out + (size_t)N * 25, s->d_reward, sizeof(float) * N);
-  memcpy(s->h_pin_out + (size_t)N * 26, s->d_done, sizeof(float) * N); memcpy(s->h_pin_out + (size_t)N * 27, s->d_info, sizeof(float) * N * 4);
-#endif
-  return 0;
+  FeedDev& F = s->F;
+  F.P = *p;
+  if (p->n_foods > 16) return fail("too many foods");
+  drop_graph(s->fused[FT_FEEDING].graph);          // the captured step refers to the previous FeedDev
+  if (!s->fused[FT_FEEDING].ready) {              // buffers are allocated once; a later init (episode reset) only refreshes their contents
+    F.male = dalloc<int>(s, N); F.food_state = dalloc<int>(s, N); F.iteration = dalloc<int>(s, N); F.task_success = dalloc<int>(s, N);
+    F.food_near = dalloc<int>(s, (size_t)N * 16);
+    F.action = dalloc<float>(s, (size_t)N * 7); F.rng = dalloc<unsigned long long>(s, N);
+    F.tremor_on = dalloc<int>(s, N); F.tremor_rest = dalloc<float>(s, (size_t)N * 4); F.tremor_amp = dalloc<float>(s, (size_t)N * 4);
+    s->F_dev = dalloc<FeedDev>(s, 1);
+    if (!s->F_dev) return fail("device allocation failed");
+  } else {
+    if (dev_zero(s, F.tremor_on, sizeof(int) * N) || dev_zero(s, F.rng, sizeof(unsigned long long) * N)) return -1;
+  }
+  if (fused_alloc(s, FT_FEEDING, 25, feeding_step_enqueue)) return -1;
+  if (h2d(s, F.male, gender_is_male, sizeof(int) * N)) return -1;
+  if (!s->F_dev || h2d(s, s->F_dev, &s->F, sizeof(FeedDev))) return fail("FeedDev upload failed");
+  s->fused[FT_FEEDING].ready = true;
+  return ag_feeding_reset_episode(s, nullptr);
 }
-int ag_feeding_step_host_end(AgSim* s, float* obs, float* reward, float* done, float* info) {
+int ag_feeding_set_tremor(AgSim* s, const int32_t* on, const float* rest, const float* amplitude) {
   DevGuard guard__(s->device);
-  if (!s->feeding) return fail("ag_feeding_init not called");
-  const int N = s->S.N;
-#ifndef AG_CPU_EMU
-  CK(cudaStreamSynchronize(s->stream));
-  CK(cudaGetLastError());
-#endif
-  memcpy(obs, s->h_pin_out, sizeof(float) * N * 25);
-  memcpy(reward, s->h_pin_out + (size_t)N * 25, sizeof(float) * N);
-  memcpy(done, s->h_pin_out + (size_t)N * 26, sizeof(float) * N);
-  if (info) memcpy(info, s->h_pin_out + (size_t)N * 27, sizeof(float) * N * 4);
-  return 0;
-}
-int ag_feeding_step_host(AgSim* s, const float* action, float* obs, float* reward, float* done, float* info) {
-  if (ag_feeding_step_host_begin(s, action)) return -1;
-  return ag_feeding_step_host_end(s, obs, reward, done, info);
+  return set_tremor(s, FT_FEEDING, 4, s->F.tremor_on, s->F.tremor_rest, s->F.tremor_amp, on, rest, amplitude);
 }
 
-// ------------------------------------------------------------------ fused BedBathingEnv path
-int ag_bathing_init(AgSim* s, const AgBathingParams* p, const int32_t* gender_is_male, const float* targets_world, const int32_t* targets_valid) {
+int ag_feeding_reset_episode(AgSim* s, const int32_t* env_mask) {
   DevGuard guard__(s->device);
+  if (need_init(s, FT_FEEDING)) return -1;
   const int N = s->S.N;
-  BathDev& B = s->B;
-  B.P = *p;
-  drop_graph(s, 1);
-  const int T = p->n_targets_max;
-  if (T <= 0 || T > 4096) return fail("bad target count");
-  for (int j = 0; j < 7; j++) if (p->arm_links[j] < 0 || p->arm_links[j] >= s->nl) return fail("bad link");
-  if (p->cloth_link < 0 || p->cloth_link >= s->nl || p->ee_link < 0 || p->ee_link >= s->nl) return fail("bad link");
-  if (!s->bathing) {
-    B.male = dalloc<int>(s, N); B.iteration = dalloc<int>(s, N); B.task_success = dalloc<int>(s, N); B.total_targets = dalloc<int>(s, N);
-    B.action = dalloc<float>(s, (size_t)N * 7);
-    B.targets = dalloc<float>(s, (size_t)T * 3 * N); B.alive = dalloc<int>(s, (size_t)T * N);
-    B.n_slots = p->human_ncol_m > p->human_ncol_f ? p->human_ncol_m : p->human_ncol_f;
-    B.dist_part = dalloc<float>(s, (size_t)(B.n_slots > 0 ? B.n_slots : 1) * N);
-    s->d_baction = dalloc<float>(s, (size_t)N * 7); s->d_bobs = dalloc<float>(s, (size_t)N * 24);
-    s->d_breward = dalloc<float>(s, N); s->d_bdone = dalloc<float>(s, N); s->d_binfo = dalloc<float>(s, (size_t)N * 4);
-    s->B_dev = dalloc<BathDev>(s, 1);
-    if (!s->B_dev || !s->d_binfo || !B.dist_part) return fail("device allocation failed");
-#ifndef AG_CPU_EMU
-    CK(cudaMallocHost((void**)&s->h_bpin_in, sizeof(float) * N * 7));
-    CK(cudaMallocHost((void**)&s->h_bpin_out, sizeof(float) * N * 30));
-#else
-    s->h_bpin_in = (float*)malloc(sizeof(float) * N * 7); s->h_bpin_out = (float*)malloc(sizeof(float) * N * 30);
-#endif
-  } else if (T != s->B.P.n_targets_max) return fail("target count changed");
-  std::vector<float> tw((size_t)T * 3 * N); std::vector<int> al((size_t)T * N), tot(N, 0), zero(N, 0);
-  for (int e = 0; e < N; e++)
-    for (int t = 0; t < T; t++) {
-      int v = targets_valid[(size_t)e * T + t] != 0;
-      al[(size_t)t * N + e] = v; tot[e] += v;
-      for (int c = 0; c < 3; c++) tw[((size_t)t * 3 + c) * N + e] = targets_world[((size_t)e * T + t) * 3 + c];
-    }
-  if (h2d(s, B.targets, tw.data(), tw.size() * sizeof(float)) || h2d(s, B.alive, al.data(), al.size() * sizeof(int))) return -1;
-  if (h2d(s, B.total_targets, tot.data(), sizeof(int) * N) || h2d(s, B.male, gender_is_male, sizeof(int) * N)) return -1;
-  if (h2d(s, B.iteration, zero.data(), sizeof(int) * N) || h2d(s, B.task_success, zero.data(), sizeof(int) * N)) return -1;
-  if (h2d(s, s->B_dev, &s->B, sizeof(BathDev))) return fail("BathDev upload failed");
-  s->bathing = true;
+  std::vector<int> fs(N), it(N), ts(N); std::vector<unsigned long long> rng(N);
+  if (d2h(s, fs.data(), s->F.food_state, sizeof(int) * N) || d2h(s, it.data(), s->F.iteration, sizeof(int) * N) ||
+      d2h(s, ts.data(), s->F.task_success, sizeof(int) * N) || d2h(s, rng.data(), s->F.rng, sizeof(unsigned long long) * N)) return -1;
+  int full = (1 << s->F.P.n_foods) - 1;
+  for (int e = 0; e < N; e++) if (!env_mask || env_mask[e]) {
+    fs[e] = full | (full << 16); it[e] = 0; ts[e] = 0;
+    if (rng[e] == 0) rng[e] = (s->F.P.seed + 0x9E3779B97F4A7C15ull * (unsigned long long)(e + 1)) | 1ull;
+  }
+  if (h2d(s, s->F.food_state, fs.data(), sizeof(int) * N) || h2d(s, s->F.iteration, it.data(), sizeof(int) * N) ||
+      h2d(s, s->F.task_success, ts.data(), sizeof(int) * N) || h2d(s, s->F.rng, rng.data(), sizeof(unsigned long long) * N)) return -1;
   return 0;
 }
+
+int ag_feeding_step_dev(AgSim* s, const float* action_dev, float* obs_dev, float* reward_dev, float* done_dev, float* info_dev) {
+  DevGuard guard__(s->device); return fused_step_dev(s, FT_FEEDING, action_dev, obs_dev, reward_dev, done_dev, info_dev); }
+int ag_feeding_step_host_begin(AgSim* s, const float* action) {
+  DevGuard guard__(s->device); return fused_step_host_begin(s, FT_FEEDING, action); }
+int ag_feeding_step_host_end(AgSim* s, float* obs, float* reward, float* done, float* info) {
+  DevGuard guard__(s->device); return fused_step_host_end(s, FT_FEEDING, obs, reward, done, info); }
+int ag_feeding_step_host(AgSim* s, const float* action, float* obs, float* reward, float* done, float* info) {
+  DevGuard guard__(s->device); return fused_step_host(s, FT_FEEDING, action, obs, reward, done, info); }
+
+// ------------------------------------------------------------------ fused BedBathingEnv path
 static int bathing_step_enqueue(AgSim* s, const float* action_dev, float* obs, float* reward, float* done, float* info) {
   const int N = s->S.N;
   KP p = kp0(); p.p0 = action_dev; p.p1 = s->B_dev;
@@ -1632,43 +1546,44 @@ static int bathing_step_enqueue(AgSim* s, const float* action_dev, float* obs, f
   LAUNCH(s, k_bath_post, N, q);
   return 0;
 }
-int ag_bathing_step_dev(AgSim* s, const float* action_dev, float* obs_dev, float* reward_dev, float* done_dev, float* info_dev) {
+int ag_bathing_init(AgSim* s, const AgBathingParams* p, const int32_t* gender_is_male, const float* targets_world, const int32_t* targets_valid) {
   DevGuard guard__(s->device);
-  if (!s->bathing) return fail("ag_bathing_init not called");
-  int rc = run_step(s, 1, bathing_step_enqueue, action_dev, obs_dev, reward_dev, done_dev, info_dev);
-#ifndef AG_CPU_EMU
-  CK(cudaGetLastError());
-#endif
-  return rc;
-}
-int ag_bathing_step_host(AgSim* s, const float* action, float* obs, float* reward, float* done, float* info) {
-  DevGuard guard__(s->device);
-  if (!s->bathing) return fail("ag_bathing_init not called");
   const int N = s->S.N;
-  memcpy(s->h_bpin_in, action, sizeof(float) * N * 7);
-#ifndef AG_CPU_EMU
-  CK(cudaMemcpyAsync(s->d_baction, s->h_bpin_in, sizeof(float) * N * 7, cudaMemcpyHostToDevice, s->stream));
-#else
-  memcpy(s->d_baction, s->h_bpin_in, sizeof(float) * N * 7);
-#endif
-  if (run_step(s, 1, bathing_step_enqueue, s->d_baction, s->d_bobs, s->d_breward, s->d_bdone, s->d_binfo)) return -1;
-#ifndef AG_CPU_EMU
-  CK(cudaMemcpyAsync(s->h_bpin_out, s->d_bobs, sizeof(float) * N * 24, cudaMemcpyDeviceToHost, s->stream));
-  CK(cudaMemcpyAsync(s->h_bpin_out + (size_t)N * 24, s->d_breward, sizeof(float) * N, cudaMemcpyDeviceToHost, s->stream));
-  CK(cudaMemcpyAsync(s->h_bpin_out + (size_t)N * 25, s->d_bdone, sizeof(float) * N, cudaMemcpyDeviceToHost, s->stream));
-  CK(cudaMemcpyAsync(s->h_bpin_out + (size_t)N * 26, s->d_binfo, sizeof(float) * N * 4, cudaMemcpyDeviceToHost, s->stream));
-  CK(cudaStreamSynchronize(s->stream));
-  CK(cudaGetLastError());
-#else
-  memcpy(s->h_bpin_out, s->d_bobs, sizeof(float) * N * 24); memcpy(s->h_bpin_out + (size_t)N * 24, s->d_breward, sizeof(float) * N);
-  memcpy(s->h_bpin_out + (size_t)N * 25, s->d_bdone, sizeof(float) * N); memcpy(s->h_bpin_out + (size_t)N * 26, s->d_binfo, sizeof(float) * N * 4);
-#endif
-  memcpy(obs, s->h_bpin_out, sizeof(float) * N * 24);
-  memcpy(reward, s->h_bpin_out + (size_t)N * 24, sizeof(float) * N);
-  memcpy(done, s->h_bpin_out + (size_t)N * 25, sizeof(float) * N);
-  if (info) memcpy(info, s->h_bpin_out + (size_t)N * 26, sizeof(float) * N * 4);
+  BathDev& B = s->B;
+  B.P = *p;
+  drop_graph(s->fused[FT_BATHING].graph);
+  const int T = p->n_targets_max;
+  if (T <= 0 || T > 4096) return fail("bad target count");
+  for (int j = 0; j < 7; j++) if (p->arm_links[j] < 0 || p->arm_links[j] >= s->nl) return fail("bad link");
+  if (p->cloth_link < 0 || p->cloth_link >= s->nl || p->ee_link < 0 || p->ee_link >= s->nl) return fail("bad link");
+  if (!s->fused[FT_BATHING].ready) {
+    B.male = dalloc<int>(s, N); B.iteration = dalloc<int>(s, N); B.task_success = dalloc<int>(s, N); B.total_targets = dalloc<int>(s, N);
+    B.action = dalloc<float>(s, (size_t)N * 7);
+    B.targets = dalloc<float>(s, (size_t)T * 3 * N); B.alive = dalloc<int>(s, (size_t)T * N);
+    B.n_slots = p->human_ncol_m > p->human_ncol_f ? p->human_ncol_m : p->human_ncol_f;
+    B.dist_part = dalloc<float>(s, (size_t)(B.n_slots > 0 ? B.n_slots : 1) * N);
+    s->B_dev = dalloc<BathDev>(s, 1);
+    if (!s->B_dev || !B.dist_part) return fail("device allocation failed");
+  } else if (T != s->B.P.n_targets_max) return fail("target count changed");
+  if (fused_alloc(s, FT_BATHING, 24, bathing_step_enqueue)) return -1;
+  std::vector<float> tw((size_t)T * 3 * N); std::vector<int> al((size_t)T * N), tot(N, 0), zero(N, 0);
+  for (int e = 0; e < N; e++)
+    for (int t = 0; t < T; t++) {
+      int v = targets_valid[(size_t)e * T + t] != 0;
+      al[(size_t)t * N + e] = v; tot[e] += v;
+      for (int c = 0; c < 3; c++) tw[((size_t)t * 3 + c) * N + e] = targets_world[((size_t)e * T + t) * 3 + c];
+    }
+  if (h2d(s, B.targets, tw.data(), tw.size() * sizeof(float)) || h2d(s, B.alive, al.data(), al.size() * sizeof(int))) return -1;
+  if (h2d(s, B.total_targets, tot.data(), sizeof(int) * N) || h2d(s, B.male, gender_is_male, sizeof(int) * N)) return -1;
+  if (h2d(s, B.iteration, zero.data(), sizeof(int) * N) || h2d(s, B.task_success, zero.data(), sizeof(int) * N)) return -1;
+  if (h2d(s, s->B_dev, &s->B, sizeof(BathDev))) return fail("BathDev upload failed");
+  s->fused[FT_BATHING].ready = true;
   return 0;
 }
+int ag_bathing_step_dev(AgSim* s, const float* action_dev, float* obs_dev, float* reward_dev, float* done_dev, float* info_dev) {
+  DevGuard guard__(s->device); return fused_step_dev(s, FT_BATHING, action_dev, obs_dev, reward_dev, done_dev, info_dev); }
+int ag_bathing_step_host(AgSim* s, const float* action, float* obs, float* reward, float* done, float* info) {
+  DevGuard guard__(s->device); return fused_step_host(s, FT_BATHING, action, obs, reward, done, info); }
 
 }  // extern "C"
 

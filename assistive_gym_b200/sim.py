@@ -47,6 +47,18 @@ class BatchSim:
         if rc != 0:
             raise RuntimeError(self.lib.ag_last_error().decode())
 
+    # ---- the fused env steps (one call: action -> obs [n, obs_dim], reward [n], done [n], info [n, 4])
+    def _step_host(self, fn, obs_dim, *action):
+        """fn(sim, [action [n, 7],] obs, reward, done, info) on host arrays; returns (obs, reward, done, info)"""
+        out = (np.empty((self.n, obs_dim), dtype=np.float32), np.empty(self.n, dtype=np.float32), np.empty(self.n, dtype=np.float32),
+               np.empty((self.n, 4), dtype=np.float32))
+        self._ck(fn(self.h, *[_p(_f32(a, (self.n, 7))) for a in action], *[_p(o) for o in out]))
+        return out
+
+    def _step_dev(self, fn, *ptrs):
+        """device pointers (ints) to action [n, 7], obs, reward, done, info; asynchronous on the sim's stream"""
+        self._ck(fn(self.h, *[C.c_void_p(p) for p in ptrs]))
+
     def close(self):
         if getattr(self, 'h', None):
             self.lib.ag_destroy(self.h)
@@ -231,15 +243,10 @@ class BatchSim:
         self._ck(self.lib.ag_bathing_init(self.h, C.byref(params), _p(g), _p(tw), _p(tv)))
 
     def bathing_step_host(self, action):
-        a = _f32(action, (self.n, 7))
-        obs = np.zeros((self.n, 24), dtype=np.float32)
-        rew, done = np.zeros(self.n, dtype=np.float32), np.zeros(self.n, dtype=np.float32)
-        info = np.zeros((self.n, 4), dtype=np.float32)
-        self._ck(self.lib.ag_bathing_step_host(self.h, _p(a), _p(obs), _p(rew), _p(done), _p(info)))
-        return obs, rew, done, info
+        return self._step_host(self.lib.ag_bathing_step_host, 24, action)
 
     def bathing_step_dev(self, action_ptr, obs_ptr, reward_ptr, done_ptr, info_ptr):
-        self._ck(self.lib.ag_bathing_step_dev(self.h, C.c_void_p(action_ptr), C.c_void_p(obs_ptr), C.c_void_p(reward_ptr), C.c_void_p(done_ptr), C.c_void_p(info_ptr)))
+        self._step_dev(self.lib.ag_bathing_step_dev, action_ptr, obs_ptr, reward_ptr, done_ptr, info_ptr)
 
     # ---- cloth (ag_cloth_*; node arrays in the PUBLIC node order of the ClothModel)
     def cloth_init(self, model, col_links, col_static, anchor_nodes, anchor_local, gravity=(0, 0, -9.81), max_contacts=1024):
@@ -287,16 +294,10 @@ class BatchSim:
         self._ck(self.lib.ag_scratch_init(self.h, C.byref(params), _p(_i32(gender_is_male)), _p(_i32(limb_link)), _p(_f32(target_local, (self.n, 3)))))
 
     def scratch_step_host(self, action):
-        a = _f32(action, (self.n, 7))
-        obs = np.empty((self.n, 30), dtype=np.float32)
-        rew = np.empty(self.n, dtype=np.float32)
-        done = np.empty(self.n, dtype=np.float32)
-        info = np.empty((self.n, 4), dtype=np.float32)
-        self._ck(self.lib.ag_scratch_step_host(self.h, _p(a), _p(obs), _p(rew), _p(done), _p(info)))
-        return obs, rew, done, info
+        return self._step_host(self.lib.ag_scratch_step_host, 30, action)
 
     def scratch_step_dev(self, action_ptr, obs_ptr, reward_ptr, done_ptr, info_ptr):
-        self._ck(self.lib.ag_scratch_step_dev(self.h, action_ptr, obs_ptr, reward_ptr, done_ptr, info_ptr))
+        self._step_dev(self.lib.ag_scratch_step_dev, action_ptr, obs_ptr, reward_ptr, done_ptr, info_ptr)
 
     # ---- camera images (ag_render)
     def render(self, eye, target, fov=60.0, width=480, height=270, env_ids=(0,), up=(0, 0, 1), near=0.01, far=100.0,
@@ -321,42 +322,25 @@ class BatchSim:
         self._ck(self.lib.ag_dressing_reset_episode(self.h, _p(_i32(mask))))
 
     def dressing_step_host(self, action):
-        a = _f32(action, (self.n, 7))
-        obs = np.empty((self.n, 24), dtype=np.float32)
-        rew = np.empty(self.n, dtype=np.float32)
-        done = np.empty(self.n, dtype=np.float32)
-        info = np.empty((self.n, 4), dtype=np.float32)
-        self._ck(self.lib.ag_dressing_step_host(self.h, _p(a), _p(obs), _p(rew), _p(done), _p(info)))
-        return obs, rew, done, info
+        return self._step_host(self.lib.ag_dressing_step_host, 24, action)
 
     def dressing_step_dev(self, action_ptr, obs_ptr, reward_ptr, done_ptr, info_ptr):
-        self._ck(self.lib.ag_dressing_step_dev(self.h, action_ptr, obs_ptr, reward_ptr, done_ptr, info_ptr))
+        self._step_dev(self.lib.ag_dressing_step_dev, action_ptr, obs_ptr, reward_ptr, done_ptr, info_ptr)
 
     def feeding_reset_episode(self, mask=None):
         self._ck(self.lib.ag_feeding_reset_episode(self.h, _p(_i32(mask))))
 
     def feeding_step_host(self, action):
-        a = _f32(action, (self.n, 7))
-        obs = np.zeros((self.n, 25), dtype=np.float32)
-        rew, done = np.zeros(self.n, dtype=np.float32), np.zeros(self.n, dtype=np.float32)
-        info = np.zeros((self.n, 4), dtype=np.float32)
-        self._ck(self.lib.ag_feeding_step_host(self.h, _p(a), _p(obs), _p(rew), _p(done), _p(info)))
-        return obs, rew, done, info
+        return self._step_host(self.lib.ag_feeding_step_host, 25, action)
 
     def feeding_step_host_begin(self, action):
-        self._host_a = _f32(action, (self.n, 7))
-        self._ck(self.lib.ag_feeding_step_host_begin(self.h, _p(self._host_a)))
+        self._ck(self.lib.ag_feeding_step_host_begin(self.h, _p(_f32(action, (self.n, 7)))))
 
     def feeding_step_host_end(self):
-        obs = np.zeros((self.n, 25), dtype=np.float32)
-        rew, done = np.zeros(self.n, dtype=np.float32), np.zeros(self.n, dtype=np.float32)
-        info = np.zeros((self.n, 4), dtype=np.float32)
-        self._ck(self.lib.ag_feeding_step_host_end(self.h, _p(obs), _p(rew), _p(done), _p(info)))
-        return obs, rew, done, info
+        return self._step_host(self.lib.ag_feeding_step_host_end, 25)
 
     def feeding_step_dev(self, action_ptr, obs_ptr, reward_ptr, done_ptr, info_ptr):
-        self._ck(self.lib.ag_feeding_step_dev(self.h, C.c_void_p(action_ptr), C.c_void_p(obs_ptr), C.c_void_p(reward_ptr),
-                                              C.c_void_p(done_ptr), C.c_void_p(info_ptr)))
+        self._step_dev(self.lib.ag_feeding_step_dev, action_ptr, obs_ptr, reward_ptr, done_ptr, info_ptr)
 
 
 class BatchSimGroup:

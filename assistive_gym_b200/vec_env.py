@@ -59,8 +59,8 @@ class AssistiveVecEnv:
         if self._standby is not None:
             self._start_standby()
         sim = self.env.id
-        self._step_dev = {'feeding': sim.feeding_step_dev, 'bed_bathing': sim.bathing_step_dev, 'dressing': sim.dressing_step_dev, 'scratch_itch': sim.scratch_step_dev}[self.task]
-        self._step_host = {'feeding': sim.feeding_step_host, 'bed_bathing': sim.bathing_step_host, 'dressing': sim.dressing_step_host, 'scratch_itch': sim.scratch_step_host}[self.task]
+        prefix = {'feeding': 'feeding', 'bed_bathing': 'bathing', 'dressing': 'dressing', 'scratch_itch': 'scratch'}[self.task]
+        self._step_dev, self._step_host = getattr(sim, prefix + '_step_dev'), getattr(sim, prefix + '_step_host')
         self._t = 0
         return obs
 

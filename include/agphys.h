@@ -214,7 +214,8 @@ int ag_feeding_reset_episode(AgSim* sim, const int32_t* env_mask);
 int ag_feeding_set_tremor(AgSim* sim, const int32_t* on, const float* rest, const float* amplitude);
 int ag_feeding_step_dev(AgSim* sim, const float* action_dev, float* obs_dev, float* reward_dev,
                         float* done_dev, float* info_dev);
-/* host-buffer variant (pinned or pageable): H2D of action, D2H of obs/reward/done/info inside */
+/* host-buffer variant (pinned or pageable): H2D of action, D2H of obs/reward/done/info inside.  `info` may be NULL, here,
+ * in ag_feeding_step_host_end and in the bathing / dressing / scratch *_step_host alike. */
 int ag_feeding_step_host(AgSim* sim, const float* action, float* obs, float* reward, float* done, float* info);
 /* the same in two halves, so that several sims (sub-batches on their own streams) overlap: `begin` stages the actions and
  * enqueues H2D + step + D2H on the sim's stream and returns, `end` waits for the stream and hands the results out */
